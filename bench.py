@@ -62,6 +62,8 @@ def parse_args():
                     help="allgather: pire_gpu_run_sharded (C ABI, NCCL all-gather of bitmap slots, overlapped); "
                          "allreduce: torch.distributed all-reduce of the zeroed full bitmap (north_star's wording, serialized)")
     ap.add_argument("--cpu-sample", type=int, default=1 << 22, help="strings in the CPU-baseline sample (per step of the reference arm)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (match bitmap, accept masks) to DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -545,6 +547,24 @@ def parity_check(res, world, bits=None, dense=1 << 22, cpu_timing=None):
             "bytes": "copied back from the HBM buffer the GPU scanned"}, cpu_record
 
 
+DUMP_MASKS = 1 << 21                 # accept masks written by --dump-outputs: all of them up to this many, else a seeded sample
+
+
+def dump_outputs(out_dir, bits, masks):
+    """What the scan hands its caller, as float64 (exact for 32-bit words): the whole match bitmap (bit i of word i // 32
+    is string i) and the accept mask of every string, or of a fixed seeded sample of DUMP_MASKS strings, with their
+    indices.  About 35 MB at the default 9.77 M strings.  At N > 1: the gathered bitmap and rank 0's masks."""
+    import numpy as np
+    import torch
+    n = masks.numel()
+    idx = np.arange(n) if n <= DUMP_MASKS else np.sort(np.random.default_rng(0).choice(n, DUMP_MASKS, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "match_bits.npy"), bits.cpu().numpy().view(np.uint32).astype(np.float64))
+    np.save(os.path.join(out_dir, "accept_mask.npy"),
+            masks[torch.from_numpy(idx).to(masks.device)].cpu().numpy().view(np.uint32).astype(np.float64))
+    np.save(os.path.join(out_dir, "accept_mask_string.npy"), idx.astype(np.float64))
+
+
 def sub_config(workload, dev, args):
     """Another BASELINE config on its own corpus, this GPU only: throughput, roofline fraction, parity."""
     import torch
@@ -675,6 +695,8 @@ def main():
     last = (step_no[0] - 1) % len(bits_all)
     bits_full = bits_all[last]
     bits_local = slot(last)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, bits_full, res.masks)
     # the scan kernel alone (CUDA events around the launches only), for the roofline
     kernel_ms = res.time_scan(min(args.steps, 10), bits_local)
     torch.cuda.synchronize()

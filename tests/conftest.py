@@ -87,13 +87,24 @@ def golden():
     return GOLDEN
 
 
-@pytest.fixture(scope="session")
-def ref():
-    """The real reference (oracle/_ref); absent when neither /root/reference nor a prebuilt copy exists."""
-    import refpire
-    if not refpire.have_ref():
-        pytest.skip("oracle/_ref/libpire_ref.so not built (needs /root/reference)")
-    return refpire.Ref()
+@pytest.hookimpl(hookwrapper=True)
+def pytest_runtest_makereport(item, call):
+    # the `ref` fixture checks its answers against the recording only for a test body that passed: a failed test has
+    # already said what went wrong, and asked only part of its questions
+    outcome = yield
+    if call.when == "call":
+        item.call_failed = outcome.get_result().failed
+
+
+@pytest.fixture
+def ref(request):
+    """The reference's answers, as recorded in tests/golden/reference_answers.json.xz (tests/refgolden.py); with
+    PIRE_REF_RECORD=<file> the real reference (oracle/_ref) answers and the recording is written to <file>."""
+    import refgolden
+    r = refgolden.GoldenRef("%s::%s" % (request.module.__name__, request.node.name), os.environ.get("PIRE_REF_RECORD"))
+    yield r
+    if not getattr(request.node, "call_failed", True):
+        r.finish()
 
 
 @pytest.fixture(scope="session")

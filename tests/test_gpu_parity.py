@@ -2,7 +2,7 @@
 
 Checkers, in order of authority:
   1. committed golden fixtures generated from the real reference;
-  2. the real reference itself (oracle/_ref/libpire_ref.so travels to the GPU box);
+  2. the real reference's answers, recorded (tests/refgolden.py);
   3. the C restatement oracle/pire_oracle.c.
 Bar: bit-exact match bits, accept masks and StateIndex for every string.
 """

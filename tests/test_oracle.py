@@ -1,7 +1,7 @@
 """The oracle (oracle/pire_oracle.c) pinned against the reference:
  * the committed golden fixtures (generated from the real reference by
    tests/golden/make_golden.py) -- always;
- * the real reference compiled from /root/reference (oracle/_ref) -- when present.
+ * the real reference's answers to the same questions, recorded (tests/refgolden.py).
 """
 import numpy as np
 import pytest
@@ -43,7 +43,7 @@ def test_oracle_rejects_bad_images():
 
 
 def test_oracle_vs_reference_live(ref):
-    """Every vector group, compiled afresh by the real reference, incl. random text."""
+    """Every vector group, compiled by the real reference, incl. random text."""
     rng = np.random.default_rng(7)
     for name, pat, opts, acc, den in VECTORS:
         sc = ref.compile(pat, opts)
